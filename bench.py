@@ -4,10 +4,12 @@ corr-lookup kernel's HBM roofline and the CPU baseline beside it.
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference|reference_gpu] [--model raft_nc_dbl|raft]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
---impl reference      the UNMODIFIED reference (baseline/_ref, installed by baseline/install_reference.sh) on the host CPU cores
+--impl reference      the UNMODIFIED reference (oracle/_ref, copied there by oracle/install_reference.py) on the host CPU cores
 --impl reference_gpu  the same reference modules in eager PyTorch on the GPU, TF32 off (SURVEY.md §0.1: "the bar"); the native
                       arm runs this leg in a subprocess (the reference's module names clash with the drop-in's) and reports it
                       as `gpu_eager_baseline`
+--dump-outputs DIR    after the timed steps, write the flows (flow_lo, flow_up; `loss` in --mode train) the last timed step
+                      returned as DIR/<name>.npy; the inputs and weights are seeded, so two builds compare output for output
 
 A "step" = one RAFT.forward over one batch of synthetic pairs (BASELINE configs[2]: batch 8 per GPU, 1024x436 padded to
 440, 32 iterations, model raft_nc_dbl = full path incl. the NCUP upsampler; configs[1]'s corr-lookup kernel is timed
@@ -25,7 +27,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.join(ROOT, "raft-ncup_b200")
-REF_CORE = os.path.join(ROOT, "baseline", "_ref", "core")        # pip-installed copy of the unmodified reference (git-ignored)
+REF_CORE = os.path.join(ROOT, "oracle", "_ref", "core")          # copy of the unmodified reference (git-ignored)
 
 import torch  # noqa: E402
 
@@ -95,7 +97,7 @@ def ref_args(dataset="sintel"):
 
 
 def reference_model(name):
-    """RAFT(args) of the unmodified reference (baseline/_ref/core/raft_nc_dbl.py:26 / raft.py:24), seed 1234 (train.py:345)."""
+    """RAFT(args) of the unmodified reference (oracle/_ref/core/raft_nc_dbl.py:26 / raft.py:24), seed 1234 (train.py:345)."""
     import importlib
     import warnings
     warnings.filterwarnings("ignore")
@@ -152,9 +154,9 @@ def host_cores():
 
 
 def cpu_reference_pairs_per_s(steps, warmup, model_name="raft_nc_dbl"):
-    """The reference's own CPU path on the host cores: RAFT(args).eval() from baseline/_ref under torch.no_grad(), fp32, all
+    """The reference's own CPU path on the host cores: RAFT(args).eval() from oracle/_ref under torch.no_grad(), fp32, all
     the cores the cgroup allows.  One step = ONE pair at the full 1024x436 / 32-iteration shape (a bounded sample of the 8-pair
-    batch: ~7 s).  Falls back to the oracle port (pinned to the reference by tests/golden) when baseline/_ref is absent.
+    batch: ~7 s).  Falls back to the oracle port (pinned to the reference by tests/golden) when oracle/_ref is absent.
     Returns (pairs/s, s/step, kind)."""
     torch.set_num_threads(host_cores())
     p1, p2 = synth_frames(1, 7)
@@ -198,7 +200,7 @@ def run_reference(args, rank):
         "dtype": "f32", "data": "synthetic",
         "config": {"workload": f"cfg2/3: 1024x436 (pad 440), 32 iters, {args.model} full path incl. the upsampler, B=1 per step "
                                "(bounded sample of the B=8 batch)", "device": "host CPU",
-                   "implementation": "unmodified reference modules from baseline/_ref" if kind == "reference" else "oracle port"},
+                   "implementation": "unmodified reference modules from oracle/_ref" if kind == "reference" else "oracle port"},
         "cpu_baseline": {"value": v, "unit": "pairs/s", "cores": cores, "kind": kind, "sample": CPU_SAMPLE},
         "e2e": {"value": v, "unit": "pairs/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}))
 
@@ -207,7 +209,7 @@ def run_reference_gpu(args):
     """SURVEY.md §0.1 / BASELINE.md §3.5: the reference's eager PyTorch path on the same B200 (cuBLAS bmm volume + grid_sample
     + cuDNN convolutions), TF32 off so that it computes what its CPU path computes.  CUDA events, warm-up, one JSON line."""
     if not use_reference_path() or not torch.cuda.is_available():
-        print(json.dumps({"impl": "reference_gpu", "unavailable": "baseline/_ref or GPU missing"}))
+        print(json.dumps({"impl": "reference_gpu", "unavailable": "oracle/_ref or GPU missing"}))
         return
     torch.backends.cudnn.allow_tf32 = False
     torch.backends.cuda.matmul.allow_tf32 = False
@@ -231,13 +233,13 @@ def run_reference_gpu(args):
     print(json.dumps({"impl": "reference_gpu", "metric": METRIC, "value": args.batch / (ms * 1e-3), "unit": "pairs/s",
                       "ms_per_step": ms, "steps": args.steps, "batch": args.batch, "model": args.model, "dtype": "f32",
                       "tf32": False, "checksum_flow_up_abs_mean": float(up.abs().mean()),
-                      "note": "unmodified reference modules (baseline/_ref) .cuda(), eager PyTorch, cudnn/matmul TF32 disabled, "
+                      "note": "unmodified reference modules (oracle/_ref) .cuda(), eager PyTorch, cudnn/matmul TF32 disabled, "
                               "inputs resident, CUDA events"}))
 
 
 def run_reference_gpu_train(args, dev):
     """The reference's own training step in eager PyTorch on the GPU (train.py:203-227 without AMP): unmodified modules from
-    baseline/_ref, train mode + freeze_bn, sequence loss (train.py:46-71 restated: train.py itself does not import), AdamW,
+    oracle/_ref, train mode + freeze_bn, sequence loss (train.py:46-71 restated: train.py itself does not import), AdamW,
     clip 1.0 — the comparator of `--mode train`."""
     B, H, W, iters = args.train_batch, 384, 512, 12
     model = reference_model(args.model).to(dev).train()
@@ -266,13 +268,13 @@ def run_reference_gpu_train(args, dev):
     print(json.dumps({"impl": "reference_gpu", "mode": "train", "metric": TRAIN_METRIC, "value": B / (ms * 1e-3), "unit": "pairs/s",
                       "ms_per_step": ms, "steps": args.steps, "batch": B, "model": args.model, "dtype": "f32", "tf32": False,
                       "loss_last": float(loss),
-                      "note": "unmodified reference modules (baseline/_ref) in eager PyTorch, cuDNN/cuBLAS TF32 disabled"}))
+                      "note": "unmodified reference modules (oracle/_ref) in eager PyTorch, cuDNN/cuBLAS TF32 disabled"}))
 
 
 def gpu_eager_baseline(args):
     """Run the reference_gpu leg in a fresh process (module names `raft_nc_dbl`, `update`, `corr`, ... clash with the drop-in)."""
     if not os.path.isdir(REF_CORE):
-        return {"unavailable": "baseline/_ref not installed (run baseline/install_reference.sh)"}
+        return {"unavailable": "oracle/_ref not installed (run oracle/install_reference.py)"}
     cmd = [sys.executable, os.path.abspath(__file__), "--impl", "reference_gpu", "--steps", "2", "--warmup", "1",
            "--batch", str(args.batch), "--model", args.model, "--mode", args.mode, "--train-batch", str(args.train_batch)]
     try:
@@ -286,6 +288,25 @@ def gpu_eager_baseline(args):
 
 def mean_ms(pairs):
     return sum(a.elapsed_time(b) for a, b in pairs) / max(len(pairs), 1)
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays):
+    """--dump-outputs: what the timed path returned in its last timed step, one DIR/<name>.npy per array (float64 stays
+    float64, anything else is stored as float32), so that two builds can be compared output for output on the same seeded
+    inputs.  Batched outputs over 64 MiB in all keep the same leading pairs of the batch."""
+    import numpy as np
+    arrays = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    arrays = {k: a if a.dtype == np.float64 else a.astype(np.float32) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        n = DUMP_BYTES // (total // min(a.shape[0] for a in arrays.values()))
+        arrays = {k: a[:n] for k, a in arrays.items()}
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(dirname, f"{k}.npy"), a)
 
 
 def run_native(args, rank, world, local_rank):
@@ -350,7 +371,7 @@ def run_native(args, rank, world, local_rank):
             flush.zero_()                                           # L2 flush between timed iterations (not timed)
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            fn()
+            out = fn()
             e1.record()
             evs.append((e0, e1))
         barrier()
@@ -359,7 +380,7 @@ def run_native(args, rank, world, local_rank):
         t = torch.tensor([dev_ms], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)                # max over ranks
-        return t.item(), wall
+        return t.item(), wall, out
 
     for _ in range(max(args.warmup, 3)):
         step_resident()
@@ -372,10 +393,12 @@ def run_native(args, rank, world, local_rank):
     eng = model.engine()
     eng.profile = {}
     native.launch_count_reset()
-    ms_total, wall = timed(step_resident, args.steps)
+    ms_total, wall, (flow_lo, flow_up) = timed(step_resident, args.steps)
     launches = native.launch_count()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"flow_lo": flow_lo, "flow_up": flow_up})    # before later calls reuse the buffers
     prof, eng.profile = eng.profile, None
-    ms_e2e, _ = timed(step_e2e, args.steps)
+    ms_e2e, _, _ = timed(step_e2e, args.steps)
     # the lookup kernel alone (in the timed region convf1 runs underneath it on a side stream): 32 back-to-back launches
     iso_ms = None
     if hasattr(eng, "lookup_resident"):
@@ -578,6 +601,8 @@ def run_train(args, rank, world, local_rank):
         evs.append((e0, e1))
     barrier()
     launches = native.launch_count()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": loss})
     ms = sum(a.elapsed_time(b) for a, b in evs)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
@@ -653,7 +678,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--mode", default="infer", choices=["infer", "train"], help="train: one optimisation step per timed step (cfg 5)")
     ap.add_argument("--train-batch", type=int, default=2, help="pairs per GPU in --mode train")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes what the native path computed: use it with --impl native")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
