@@ -187,7 +187,10 @@ typedef struct {
 } rnc_conv_umma_desc;
 
 /* Pixel tiles (128 output pixels each) a layer of this shape is cut into: a tile-blocked tensor with ld channels has
- * rnc_conv_umma_tiles(...) * ld * 128 floats; the tiling depends on (kh, kw, stride, H, W, flags & RNC_CONV_NO_HALO) only. */
+ * rnc_conv_umma_tiles(...) * ld * 128 floats; the tiling depends on (kh, kw, stride, H, W, flags & RNC_CONV_NO_HALO) only.
+ * Tile shape TW x TH px (stride 1, no RNC_CONV_NO_HALO): 128 x 1 if kw > 1 and W > 64; 16 x 8 if kw == 1 < kh, W >= 16 and
+ * H >= 8; otherwise (and for stride 2 or RNC_CONV_NO_HALO) TW = the smallest power of two >= W in [8, 128], TH = 128 / TW.
+ * Tile t = (b * ceil(H/TH) + ty) * ceil(W/TW) + tx holds pixel (y, x) = (ty*TH + r / TW, tx*TW + r % TW) at row r. */
 long long rnc_conv_umma_tiles(int kh, int kw, int stride, int B, int H, int W, int flags);
 int rnc_conv2d_umma_fwd(const rnc_conv_umma_desc* desc, void* stream);
 
