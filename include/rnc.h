@@ -33,7 +33,7 @@ typedef enum {
 } rnc_status;
 
 /* Library identity / diagnostics. */
-int rnc_abi_version(void);                 /* bumps on any signature change (now 10) */
+int rnc_abi_version(void);                 /* bumps on any signature change (now 11) */
 const char* rnc_build_info(void);          /* e.g. "sm_100a nvcc 12.9" */
 const char* rnc_status_string(int status);
 int rnc_last_cuda_error(void);             /* cudaError_t of the last failed launch on this thread */
@@ -352,7 +352,8 @@ int rnc_nconv2d_bwd(const float* data, const float* conf, const float* weight, c
                     void* stream);
 
 /* ------------------------------------------------------------------------------------------------
- * Training path (train.py:203-227; SURVEY.md §8f-3, Appendix G): backward kernels, exact fp32.
+ * Training path (train.py:203-227; SURVEY.md §8f-3, Appendix G): backward kernels, exact fp32, and the TF32x3 tensor-core
+ * form of the convolution weight gradient.
  *
  * Gradient of CorrBlock.__call__ (core/corr.py:23-44; the reference back-propagates through the stored 4-D pyramid) w.r.t.
  * the feature maps.  coords are detached (raft_nc_dbl.py:149): no gradient flows to them.
@@ -373,6 +374,20 @@ int rnc_pyramid_pool_bwd(float* g_f2_pyr, int B, int D, int H, int W, int levels
  * The data gradient is rnc_conv2d_cl_fwd on gy (zero-dilated for stride 2) with the flipped, transposed weights. */
 int rnc_conv2d_cl_wgrad(const float* x, int ldx, int cin, const float* gy, int ldg, int cout, int B, int Hin, int Win,
                         int kh, int kw, int stride, float* gw, int ldw, float* gb, void* stream);
+
+/* The same gradient on the tensor cores (tcgen05 kind::tf32, TF32x3 like RNC_CONV_TF32: gy_hi*x_hi + gy_hi*x_lo + gy_lo*x_hi,
+ * ~2^-21 per product with fp32's exponent range).  Same arguments and accumulation contract as rnc_conv2d_cl_wgrad, plus:
+ *   workspace : rnc_conv2d_umma_wgrad_workspace_bytes(...) bytes of device memory, 16-byte aligned, caller-owned, contents
+ *               irrelevant: the TF32 hi/lo planes of x and gy, transposed to channel-major [B][C][H][W'] so that the pixels
+ *               (the GEMM's K) are contiguous; the bias gradient is summed by the same pass over gy
+ * No TMEM accumulation runs over more than 512 pixels (the tensor core truncates on every accumulate): each chunk is drained
+ * into fp32 registers and each work item (co tile, ci tile, tap, pixel range) adds its partial sums with one atomic per element.
+ * Returns RNC_ERR_WORKSPACE if workspace_bytes is too small, RNC_ERR_UNSUPPORTED for problems beyond the kernel's index
+ * ranges; nothing is launched when an argument is rejected. */
+size_t rnc_conv2d_umma_wgrad_workspace_bytes(int cin, int cout, int B, int Hin, int Win, int kh, int kw, int stride);
+int rnc_conv2d_umma_wgrad(const float* x, int ldx, int cin, const float* gy, int ldg, int cout, int B, int Hin, int Win,
+                          int kh, int kw, int stride, float* gw, int ldw, float* gb,
+                          void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

@@ -88,7 +88,7 @@ using namespace rnc;
 
 extern "C" {
 
-int rnc_abi_version(void) { return 10; }
+int rnc_abi_version(void) { return 11; }
 const char* rnc_build_info(void) { return "librnc sm_100a (CUDA " RNC_STR_CUDA ")"; }
 const char* rnc_status_string(int s) {
   switch (s) {

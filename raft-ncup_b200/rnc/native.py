@@ -10,7 +10,7 @@ import threading
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("RNC_LIB") or os.path.join(_HERE, "librnc.so")      # RNC_LIB: developer override (variant builds)
-ABI_VERSION = 10
+ABI_VERSION = 11
 CONV_NO_HALO, CONV_BASE_OFFSET, CONV_SPLIT_N, CONV_NO_PAIR, CONV_AUX_BLOCKED, CONV_OUT_BLOCKED, CONV_TF32, CONV_WINDOW = 1, 2, 4, 8, 16, 32, 64, 128   # rnc_conv_umma_desc.flags
 
 (EPI_LINEAR, EPI_RELU, EPI_SIGMOID, EPI_GRU_ZR, EPI_GRU_Q, EPI_RELU_FLOW, EPI_RELU_ADD_RELU, EPI_TANH_RELU,
@@ -104,6 +104,8 @@ SIGNATURES = {
     "rnc_corr_lookup_bwd": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
     "rnc_pyramid_pool_bwd": (_i, [_vp, _i, _i, _i, _i, _i, _vp]),
     "rnc_conv2d_cl_wgrad": (_i, [_vp, _i, _i, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _i, _vp, _vp]),
+    "rnc_conv2d_umma_wgrad_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i, _i, _i, _i, _i]),
+    "rnc_conv2d_umma_wgrad": (_i, [_vp, _i, _i, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _i, _vp, _vp, C.c_size_t, _vp]),
     "rnc_nconv2d_bwd_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i]),
     "rnc_nconv2d_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _f, _vp, _vp, _vp, _vp, C.c_size_t, _vp]),
 }

@@ -56,6 +56,9 @@ def _conv_mode():
                       survive; 112 ms per step, ill-conditioned parameters (cnet.conv1) move to 5e-3
       umma            fp16 hi/lo split operands (the inference kernels): output gradients underflow the split's normal range —
                       per-parameter gradient errors of 5e-3 (forward only) to 4e-2 (with RNC_TRAIN_DGRAD=umma)
+    The weight gradient runs on the CUDA cores (rnc_conv2d_cl_wgrad) unless RNC_TRAIN_WGRAD=tf32 qualifies the tf32 form: then
+    the layers _wgrad_umma_ok names run it as rnc_conv2d_umma_wgrad (tcgen05 TF32x3, K = pixels in chunks of 512), so that every
+    wide convolution of the step runs on the tensor cores.  RNC_TRAIN_WGRAD has no effect under ffma or umma.
     Parity first: the default is the exact path; the tensor-core forms are opt-in and reported beside it by bench.py."""
     import os
     return os.environ.get("RNC_TRAIN_CONV", "ffma")
@@ -73,6 +76,17 @@ def _umma_ok(eng, Cx, cout, dgrad=False):
     if dgrad and os.environ.get("RNC_TRAIN_DGRAD", "ffma") != "umma":
         return None
     return "f16" if Cx % 8 == 0 and Cx >= 32 and cout >= 32 else None
+
+
+def _wgrad_umma_ok(eng, Cx, cout):
+    """Does this layer's weight gradient run on the tensor cores (rnc_conv2d_umma_wgrad)?  Only when RNC_TRAIN_WGRAD=tf32 and the
+    layer's forward runs in the TF32 form.  The rule is a function of the layer's shape: narrow layers (FlowHead.conv2 256->2,
+    Simple.out 32->2, the 4-channel 7x7 stems and convf1) would fill a fraction of a 128 x N tile and stay on the CUDA cores;
+    every layer it sends to the tensor cores is faster there at config 5 (tools/wgrad_probe.py, profiles/r03_wgrad.json)."""
+    import os
+    if os.environ.get("RNC_TRAIN_WGRAD", "ffma") != "tf32" or _umma_ok(eng, Cx, cout) != "tf32":
+        return False
+    return cout >= 32 and Cx >= 16
 
 
 class _WeightsTF32:
@@ -216,8 +230,15 @@ class ConvCL(torch.autograd.Function):
             if ctx.needs_input_grad[1] or (ctx.has_bias and ctx.needs_input_grad[2]):
                 gwp = torch.zeros(kh * kw, Cx, cout, dtype=torch.float32, device=x.device)
                 gbp = torch.zeros(cout, dtype=torch.float32, device=x.device) if ctx.has_bias else None
-                native.check(eng.L.rnc_conv2d_cl_wgrad(_ptr(x), Cx, Cx, _ptr(gy), ldg, cout, B, H, W, kh, kw, ctx.stride,
-                                                       _ptr(gwp), cout, _ptr(gbp), _stream()), "conv2d_cl_wgrad")
+                if _wgrad_umma_ok(eng, Cx, cout):
+                    nbytes = eng.L.rnc_conv2d_umma_wgrad_workspace_bytes(Cx, cout, B, H, W, kh, kw, ctx.stride)
+                    ws = torch.empty((nbytes + 15) // 16 * 4, dtype=torch.float32, device=x.device)
+                    native.check(eng.L.rnc_conv2d_umma_wgrad(_ptr(x), Cx, Cx, _ptr(gy), ldg, cout, B, H, W, kh, kw, ctx.stride,
+                                                             _ptr(gwp), cout, _ptr(gbp), _ptr(ws), ws.numel() * 4, _stream()),
+                                 "conv2d_umma_wgrad")
+                else:
+                    native.check(eng.L.rnc_conv2d_cl_wgrad(_ptr(x), Cx, Cx, _ptr(gy), ldg, cout, B, H, W, kh, kw, ctx.stride,
+                                                           _ptr(gwp), cout, _ptr(gbp), _stream()), "conv2d_cl_wgrad")
                 gw = gwp.view(kh, kw, Cx, cout)[:, :, :cin].permute(3, 2, 0, 1).contiguous()
                 gb = gbp
         return gx, gw, gb, None
